@@ -1,8 +1,14 @@
 #!/usr/bin/env python
 """bench.py -- the driver's measurement contract for the k-mer hot path.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes what the timed path hands its caller after the last of the K timed steps (and the final
+all-reduce), as float64 .npy files: hist.npy (the int64 histogram the K steps accumulate into) and status.npy (the
+status words).  The inputs depend only on the arguments, so two builds run with the same arguments can be compared
+file by file.  A histogram of more than 2^21 bins is written as a fixed, seeded sample of 2^21 bins, with their
+indices in hist_index.npy, which keeps the dump under 64 MB.
 
 A "step" is one pass of the fused hot path (FASTQ chunk bytes -> 2-bit codes -> k=31 rolling hash -> bincount) over
 one batch of synthetic 150 bp reads that is already resident in HBM (BASELINE.json configs[1]: 10 M x 150 bp per GPU,
@@ -15,7 +21,7 @@ synchronize on both sides, max over ranks.
 The JSON line also carries
   roofline      achieved algorithmic GB/s of the dominant kernel (event-timed per launch) vs the measured HBM peak
   headline_2^24 the same workload into 2^24 buckets (SURVEY 8d's default for the hashed-bucket extension)
-  extra         BASELINE configs 3 (100 M reads, minimizers), 4 (sacCer3.fa, k=21), the materialising get_kmers mode,
+  extra         BASELINE configs 3 (100 M reads, minimizers), 4 (a sample of sacCer3.fa, k=21), the materialising get_kmers mode,
                 k=5 exact; each min/median over >= 10 repetitions (3 for the 100 M-read one)
   oracle_check  the 10 M-read headline table compared bin by bin with oracle/kmer_oracle.c (untimed)
   e2e           the same metric through the host-buffer C-ABI call (pinned host chunk -> sliced H2D overlapped with
@@ -61,6 +67,7 @@ def parse_args():
     ap.add_argument("--no-extra", action="store_true", help="skip the secondary configurations")
     ap.add_argument("--config3-reads", type=int, default=100_000_000)
     ap.add_argument("--cpu-sample-reads", type=int, default=200_000)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the timed path's outputs as DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -210,6 +217,23 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+DUMP_MAX_BINS = 1 << 21
+
+
+def dump_outputs(out_dir, hist, status):
+    """hist.npy and status.npy as float64 (exact: counts stay far below 2^53); a histogram of more than DUMP_MAX_BINS
+    bins as the same seeded sample of bins on every run, indices in hist_index.npy."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    h = hist.cpu().numpy()
+    if h.size > DUMP_MAX_BINS:
+        idx = np.sort(np.random.default_rng(0).choice(h.size, DUMP_MAX_BINS, replace=False))
+        np.save(os.path.join(out_dir, "hist_index.npy"), idx.astype(np.float64))
+        h = h[idx]
+    np.save(os.path.join(out_dir, "hist.npy"), h.astype(np.float64))
+    np.save(os.path.join(out_dir, "status.npy"), status.cpu().numpy().astype(np.float64))
+
+
 def timed(fn, reps, warm=2):
     """min / median of `reps` event-timed calls (ms)."""
     import torch
@@ -317,6 +341,8 @@ def main():
     ms_per_step = elapsed_ms / args.steps
     value = world * n * READ_LEN / (ms_per_step * 1e-3) / 1e9
     assert int(hist.sum().item()) == world * args.steps * n * per_read
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, hist, status)
     # clocks of every GPU of the box (one sampler), gathered as text
     clocks_all = None
     if local_rank == 0:
@@ -428,7 +454,7 @@ def main():
             del starts, lens, offsets, out
         except Exception as exc:  # pragma: no cover
             extra["materialised_get_kmers_k31"] = {"error": repr(exc)}
-        # ---- BASELINE configs[3]: sacCer3.fa whole genome, k=21 (long ragged rows) ---------------------------------------
+        # ---- BASELINE configs[3]: every sacCer3 chromosome (50 kbases each), k=21 (long ragged rows) -------------------
         try:
             extra["config4_sacCer3_k21"] = bench_saccer3(dev, peak)
         except Exception as exc:  # pragma: no cover
@@ -524,14 +550,15 @@ def main():
 
 
 def bench_saccer3(dev, peak):
-    """BASELINE configs[3]: tests/golden/sacCer3.fa.gz (the reference's own example_data file) through the kept API:
-    bnp.open(...).read_chunks() -> count_kmers_hashed(k=21, 2^24 buckets); plus the device-only time of the count."""
+    """BASELINE configs[3] in miniature: tests/golden/sacCer3_sample.fa.gz (the first 50 kbases of every chromosome of
+    the reference's example_data/sacCer3.fa) through the kept API: bnp.open(...).read_chunks() ->
+    count_kmers_hashed(k=21, 2^24 buckets); plus the device-only time of the count."""
     import gzip
     import tempfile
     import numpy as np
     import torch
     import bionumpy_b200 as bnp
-    src = os.path.join(ROOT, "tests", "golden", "sacCer3.fa.gz")
+    src = os.path.join(ROOT, "tests", "golden", "sacCer3_sample.fa.gz")
     raw = gzip.open(src).read()
     tmp = tempfile.NamedTemporaryFile(suffix=".fa", delete=False)
     tmp.write(raw)
@@ -562,7 +589,8 @@ def bench_saccer3(dev, peak):
                 "api_ms_median": round(statistics.median(ts) * 1e3, 2), "api_Gbases/s": round(n_bases / statistics.median(ts) / 1e9, 3),
                 "count_only_ms_median": round(med, 3), "count_only_Gbases/s": round(n_bases / med / 1e6, 2),
                 "count_only_frac_of_hbm_roofline": round((n_bases + 8 * B) / (med * 1e-3) / 1e9 / peak, 4),
-                "note": "17 rows of up to 1.5 Mbases; bit-exact check incl. np.unique in tests/test_gpu_round2.py::test_saccer3"}
+                "note": "17 rows of 50 kbases; bit-exact check incl. np.unique in "
+                        "tests/test_gpu_round2.py::test_saccer3_whole_genome_k21"}
     finally:
         os.unlink(tmp.name)
 

@@ -138,30 +138,31 @@ def test_two_devices_one_process():
 
 
 def test_saccer3_whole_genome_k21(bnp, tmp_path):
-    """BASELINE configs[3] on the reference's own example_data/sacCer3.fa (shipped gzipped under tests/golden):
-    multi-line FASTA -> 17 long rows -> k=21 hashes.  Bucketed histogram (2^24) AND the exact distinct-k-mer table
-    (np.unique) against the oracle (SURVEY 8d)."""
+    """BASELINE configs[3] in miniature on every chromosome of the reference's example_data/sacCer3.fa, each cut to
+    its first 50 kbases (tests/golden/sacCer3_sample.fa.gz): multi-line FASTA -> 17 long rows -> k=21 hashes.
+    Bucketed histogram (2^24) AND the exact distinct-k-mer table (np.unique) against the oracle (SURVEY 8d)."""
     import gzip
     import os
-    raw = gzip.open(os.path.join(os.path.dirname(__file__), "golden", "sacCer3.fa.gz")).read()
-    assert len(raw) == 12400379
+    raw = gzip.open(os.path.join(os.path.dirname(__file__), "golden", "sacCer3_sample.fa.gz")).read()
+    assert len(raw) == 867596
     path = tmp_path / "sacCer3.fa"
     path.write_bytes(raw)
     # oracle: the reference's multi-line split, encode, hash
     whole = np.frombuffer((raw if raw.endswith(b"\n") else raw + b"\n") + b">", dtype=np.uint8)
     size, hs, hl, flat, seq_lens = oracle.multiline_fasta_split(whole)
-    assert seq_lens.size == 17 and int(seq_lens.sum()) == 12157105
+    assert seq_lens.size == 17 and int(seq_lens.sum()) == 850455
     codes = oracle.encode_flat(flat, oracle.alphabet_lut("ACGT"))
     want_h, want_lens = oracle.get_kmers(codes, seq_lens, 21)
     B = 1 << 24
     want_hist = oracle.count_bucketed_flat(want_h, B)
     # ours, through bnp.open in chunks and as one buffer
     hist = torch.zeros(B, dtype=torch.int64, device="cuda")
-    n_entries = 0
-    for chunk in bnp.open(str(path)).read_chunks(min_chunk_size=3_000_000):
+    n_entries, n_chunks = 0, 0
+    for chunk in bnp.open(str(path)).read_chunks(min_chunk_size=200_000):
         hist += bnp.count_kmers_hashed(chunk.sequence, 21, B)
         n_entries += len(chunk)
-    assert n_entries == 17
+        n_chunks += 1
+    assert n_entries == 17 and n_chunks > 1
     assert np.array_equal(hist.cpu().numpy(), want_hist)
     chunk = bnp.open(str(path)).read()
     kmers = bnp.get_kmers(bnp.change_encoding(chunk.sequence, bnp.DNAEncoding), 21)
@@ -212,18 +213,18 @@ def test_open_ingest_paths_count_like_the_oracle(bnp, tmp_path, kind, min_chunk_
 
 
 def test_indexed_fasta_on_saccer3(bnp, tmp_path):
-    """io/indexed_fasta.py:61-206 on the reference's own sacCer3.fa: contig lengths, a whole contig, random intervals
-    (line ends skipped on the device) against the oracle's restatement; k-mers of the intervals."""
+    """io/indexed_fasta.py:61-206 on the sample of the reference's sacCer3.fa: contig lengths, a whole contig, random
+    intervals (line ends skipped on the device) against the oracle's restatement; k-mers of the intervals."""
     import gzip
     import os
-    raw = gzip.open(os.path.join(os.path.dirname(__file__), "golden", "sacCer3.fa.gz")).read()
+    raw = gzip.open(os.path.join(os.path.dirname(__file__), "golden", "sacCer3_sample.fa.gz")).read()
     path = tmp_path / "sacCer3.fa"
     path.write_bytes(raw)
     data = np.frombuffer(raw, dtype=np.uint8)
     idx = oracle.fasta_index(data)
     fa = bnp.IndexedFasta(str(path))
     assert fa.get_contig_lengths() == {k: v["rlen"] for k, v in idx.items()} and len(idx) == 17
-    assert sum(fa.get_contig_lengths().values()) == 12157105
+    assert sum(fa.get_contig_lengths().values()) == 850455
     chrom = fa["chrIII"]
     assert chrom.raw().cpu().numpy().tobytes() == oracle.indexed_fasta_interval(data, idx["chrIII"], 0, idx["chrIII"]["rlen"]).tobytes()
     rng = np.random.default_rng(2)
