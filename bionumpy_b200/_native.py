@@ -40,6 +40,8 @@ SIGNATURES = {
     "bnpk_line_split": (_i, [_vp, _sz, _i, _i, _i, _u8, _i, _i, _vp, _vp, _sz, _vp, _vp, _sz, _vp]),
     "bnpk_chunk_kmer_count": (_i, [_vp, _sz, _sz, _sz, _i, _i, _u8, _i, _i, _i, _vp, _i, _i, _i64, _i, _vp,
                                    _vp, _vp, _sz, _vp]),
+    "bnpk_chunk_kmer_count_canonical": (_i, [_vp, _sz, _sz, _sz, _i, _i, _u8, _i, _i, _i, _vp, _i, _i, _i64, _i, _vp,
+                                             _vp, _vp, _sz, _vp]),
     "bnpk_row_offsets": (_i, [_vp, _sz, _i, _vp, _vp, _sz, _vp]),
     "bnpk_rows_encode": (_i, [_vp, _sz, _vp, _vp, _sz, _i, _vp, _vp, _vp, _vp, _vp]),
     "bnpk_rows_kmer_hash": (_i, [_vp, _sz, _vp, _vp, _sz, _i, _vp, _i, _vp, _vp, _vp, _vp]),

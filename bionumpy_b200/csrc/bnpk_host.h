@@ -40,10 +40,17 @@ void profile_after(cudaStream_t st);
 size_t tile_workspace_bytes(size_t n);
 bool use_smem_hist(int64_t n_bins, int hist_mode);
 
+// the complement of a 2-bit code as an XOR pattern over a whole hash (complement_xor 1..3, see canonical_hash)
+inline uint64_t canon_pattern(int complement_xor) {
+    return complement_xor == 3 ? ~0ull : complement_xor == 2 ? 0xAAAAAAAAAAAAAAAAull : 0x5555555555555555ull;
+}
+
+// canon_xor != 0: count canonical k-mers (window must be 0)
 int chunk_kmer_count_impl(const uint8_t *chunk, size_t n, size_t slice_begin, size_t slice_end, int final_slice,
                           int lpe, uint8_t header_char, int check_plus, int trim_cr, int enc_mode,
                           const uint8_t *lut256, int k, int window, int64_t n_bins, int hist_mode, int64_t *hist,
-                          int64_t *status, void *workspace, size_t workspace_bytes, cudaStream_t st);
+                          int64_t *status, void *workspace, size_t workspace_bytes, cudaStream_t st,
+                          uint64_t canon_xor = 0);
 
 int line_split_impl(const uint8_t *chunk, size_t n, int lpe, int field_line, int start_offset, uint8_t header_char,
                     int check_plus, int trim_cr, int64_t *starts, int32_t *lens, size_t max_rows, int64_t *status,
@@ -53,6 +60,6 @@ int line_split_impl(const uint8_t *chunk, size_t n, int lpe, int field_line, int
 // of a trailing incomplete entry
 int count_fixups_impl(const uint8_t *chunk, size_t n, int lpe, int enc_mode, const uint8_t *lut256, int k,
                       int window, int64_t n_bins, int64_t *hist, int64_t *status, const uint64_t *deferred_count,
-                      const uint64_t *deferred, size_t deferred_cap, cudaStream_t st);
+                      const uint64_t *deferred, size_t deferred_cap, cudaStream_t st, uint64_t canon_xor = 0);
 
 }  // namespace bnpk

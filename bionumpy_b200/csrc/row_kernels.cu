@@ -234,7 +234,7 @@ __global__ void uncount_kernel(const RowArgs a) {
     ht.n_bins = a.n_bins;
     ht.mask = (a.n_bins & (a.n_bins - 1)) == 0 ? a.n_bins - 1 : 0;
     ht.delta = ~0ull;                                          // -1
-    ht.canon_xor = 0;
+    ht.canon_xor = a.canon_xor;                                // the values the fused pass counted
     uint64_t produced = 0;
     // the BAD_BASE slot must not be touched by this row: point validation at a scratch word
     RowArgs b = a;
@@ -360,11 +360,12 @@ static int launch_uncount(const RowArgs &a, int enc_mode, cudaStream_t st) {
 
 int count_fixups_impl(const uint8_t *chunk, size_t n, int lpe, int enc_mode, const uint8_t *lut256, int k,
                       int window, int64_t n_bins, int64_t *hist, int64_t *status, const uint64_t *deferred_count,
-                      const uint64_t *deferred, size_t deferred_cap, cudaStream_t st) {
+                      const uint64_t *deferred, size_t deferred_cap, cudaStream_t st, uint64_t canon_xor) {
     RowArgs a{};
     a.base = chunk; a.base_bytes = n; a.lut = lut256; a.k = k; a.window = window;
     a.n_bins = (uint64_t)n_bins; a.hist = (unsigned long long *)hist; a.status = status;
     a.deferred_count = deferred_count; a.deferred = deferred; a.deferred_cap = deferred_cap; a.lpe = lpe;
+    a.canon_xor = canon_xor;                                   // long rows and the un-count count canonical values too
     // long rows: a modest fixed grid; the kernel reads the row count on the device
     const size_t est = (size_t)sm_count() * kRowWarps * 2;
     int rc = window ? launch_rows_enc<RM_COUNT_MIN, false, true>(a, enc_mode, est, st)
@@ -444,10 +445,6 @@ int bnpk_rows_kmer_count(const uint8_t *base, size_t base_bytes, const int64_t *
                   : launch_rows_enc<RM_COUNT_MIN, false, false>(a, enc_mode, n_rows, st);
     return sm ? launch_rows_enc<RM_COUNT, true, false>(a, enc_mode, n_rows, st)
               : launch_rows_enc<RM_COUNT, false, false>(a, enc_mode, n_rows, st);
-}
-
-static uint64_t canon_pattern(int complement_xor) {
-    return complement_xor == 3 ? ~0ull : complement_xor == 2 ? 0xAAAAAAAAAAAAAAAAull : 0x5555555555555555ull;
 }
 
 int bnpk_rows_kmer_hash_canonical(const uint8_t *base, size_t base_bytes, const int64_t *starts, const int32_t *lens,

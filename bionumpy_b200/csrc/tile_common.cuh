@@ -28,6 +28,7 @@ struct TileArgs {
     uint64_t n_bins;
     unsigned long long *hist;
     uint32_t *hist32;              // optional 32-bit scratch table in the workspace (large global tables), else null
+    uint64_t canon_xor;            // != 0: canonical k-mers, the complement as an XOR pattern (canon_pattern)
 };
 
 // 256-bit streaming load (sm_100: LDG.E.256), read-only path, no L1 allocation
@@ -190,5 +191,7 @@ int launch_tma_count(const TileArgs &a, int enc_mode, bool smem_hist, cudaStream
 int launch_ws_count(const TileArgs &a, int enc_mode, bool smem_hist, cudaStream_t st);
 bool wsm_count_eligible(const TileArgs &a, bool smem_hist);
 int launch_wsm_count(const TileArgs &a, int enc_mode, bool smem_hist, cudaStream_t st);
+bool wsc_count_eligible(const TileArgs &a, bool smem_hist);
+int launch_wsc_count(const TileArgs &a, int enc_mode, bool smem_hist, cudaStream_t st);
 
 }  // namespace bnpk

@@ -98,6 +98,7 @@ __global__ void __launch_bounds__(kCtaThreads, MODE == 0 ? 4 : 3) tile_kernel(co
     ht.n_bins = a.n_bins;
     ht.mask = (a.n_bins & (a.n_bins - 1)) == 0 ? a.n_bins - 1 : 0;
     ht.delta = 1ull;
+    ht.canon_xor = a.canon_xor;
     uint64_t acc_bases = 0, acc_values = 0;     // per-thread statistics, flushed once
     // lines_per_entry is a power of two (1, 2 or 4): phases and entry indices are masks and shifts
     const uint32_t ls = (uint32_t)a.lpe_shift, pm = (1u << ls) - 1u;
@@ -312,7 +313,7 @@ __global__ void __launch_bounds__(kCtaThreads, MODE == 0 ? 4 : 3) tile_kernel(co
                 int s_hi = n_rows_tile;
                 if (round != n_rounds - 1) s_hi = min(s_hi, (int)((win_lo + kNlStep - (int)jr0 + (int)pm) >> ls));
                 const uint64_t kmask = (1ull << (2 * a.k)) - 1;
-                const bool fast = ht.mask && ht.mask <= 0x3FFFFFFFull;
+                const bool fast = ht.mask && ht.mask <= 0x3FFFFFFFull && !ht.canon_xor;   // the minimum needs every bit
                 const uint32_t m32x4 = (uint32_t)(ht.mask & kmask) << 2;         // byte-offset mask into the table
                 const uint32_t need_bits = (uint32_t)__popcll(ht.mask & kmask);  // stream bits one table index needs
                 constexpr int kGroups = MINIMIZER ? kCtaWarps : kCtaThreads / 4;  // rows handled concurrently
@@ -409,8 +410,14 @@ __global__ void __launch_bounds__(kCtaThreads, MODE == 0 ? 4 : 3) tile_kernel(co
                             for (int p0 = sub * 32; p0 < npos; p0 += 128) {
                                 const int n_here = min(32, npos - p0);
                                 acc_values += (uint64_t)n_here;
-                                for (int j = 0; j < n_here; ++j)
-                                    hist_add<SMEM_HIST>(ht, stream_64(s_codes, (uint32_t)(b0 + p0 + j)) & kmask);
+                                for (int j = 0; j < n_here; ++j) {
+                                    uint64_t h = stream_64(s_codes, (uint32_t)(b0 + p0 + j)) & kmask;
+                                    if (ht.canon_xor) h = canonical_hash(h, a.k, ht.canon_xor);
+                                    if (!SMEM_HIST && a.hist32)       // canonical counts into 2^22..2^24 bins
+                                        atomicAdd(a.hist32 + (ht.mask ? (h & ht.mask) : (h % ht.n_bins)), 1u);
+                                    else
+                                        hist_add<SMEM_HIST>(ht, h);
+                                }
                             }
                         }
                     }
@@ -511,14 +518,26 @@ static int tile_kernel_choice() {
 }
 static bool tma_kernel_allowed() { return tile_kernel_choice() != 0; }
 
+// the kernel a fused count of a global table goes to writes the 32-bit scratch table (a.hist32) when it gets one: the
+// tma / ws kernels, and for canonical k-mers tile_kernel (global canonical tables always go there)
+static bool count_takes_scratch32(const TileArgs &a, bool smem_hist) {
+    if (a.canon_xor) return !smem_hist;
+    return tma_kernel_allowed() && tma_count_eligible(a, smem_hist);
+}
+
 static int launch_count(const TileArgs &a, int enc_mode, bool smem_hist, cudaStream_t st) {
-    if (tma_kernel_allowed() && tile_kernel_choice() != 1 && wsm_count_eligible(a, smem_hist))
+    if (a.canon_xor) {
+        // canonical k-mers: the wsc build for CTA-private tables of up to 2^14 bins, the register-staged kernel for the
+        // rest (the round-1 kernel has no canonical build)
+        if (tma_kernel_allowed() && wsc_count_eligible(a, smem_hist)) return launch_wsc_count(a, enc_mode, smem_hist, st);
+    } else if (tma_kernel_allowed() && tile_kernel_choice() != 1 && wsm_count_eligible(a, smem_hist)) {
         return launch_wsm_count(a, enc_mode, smem_hist, st);          // minimizers, windows of up to 12 k-mers
-    if (tma_kernel_allowed() && tma_count_eligible(a, smem_hist))
+    } else if (tma_kernel_allowed() && tma_count_eligible(a, smem_hist)) {
         // the warp-specialised kernel for CTA-private tables; global tables are bound by L2 atomics, where the round-1
         // kernel's 21 row warps per SM keep more of them in flight (2^24 bins: 6.6 ms against 9.3 ms)
         return (tile_kernel_choice() == 1 || (!smem_hist && tile_kernel_choice() != 3)) ? launch_tma_count(a, enc_mode, smem_hist, st)
                                                                                        : launch_ws_count(a, enc_mode, smem_hist, st);
+    }
     switch (enc_mode) {
         case BNPK_ENC_ASCII_ACGT: return launch_count_enc<BNPK_ENC_ASCII_ACGT>(a, smem_hist, st);
         case BNPK_ENC_ASCII_ACTG: return launch_count_enc<BNPK_ENC_ASCII_ACTG>(a, smem_hist, st);
@@ -555,8 +574,9 @@ bool use_smem_hist(int64_t n_bins, int hist_mode) {
 int chunk_kmer_count_impl(const uint8_t *chunk, size_t n, size_t slice_begin, size_t slice_end, int final_slice,
                           int lpe, uint8_t header_char, int check_plus, int trim_cr, int enc_mode,
                           const uint8_t *lut256, int k, int window, int64_t n_bins, int hist_mode, int64_t *hist,
-                          int64_t *status, void *workspace, size_t workspace_bytes, cudaStream_t st) {
+                          int64_t *status, void *workspace, size_t workspace_bytes, cudaStream_t st, uint64_t canon_xor) {
     if (k < 1 || k > 31) return set_err(BNPK_E_K, "k must be larger than 0 and smaller than 32");
+    if (canon_xor != 0 && window != 0) return set_err(BNPK_E_BADARG, "canonical minimizers are not implemented");
     if (window != 0 && window < k) return set_err(BNPK_E_WINDOW, "kmer size must be smaller than window size");
     if (window > 1024) return set_err(BNPK_E_WINDOW, "window_size above 1024 is not supported");
     if (n_bins < 1) return set_err(BNPK_E_BINS, "n_bins must be positive");
@@ -582,6 +602,7 @@ int chunk_kmer_count_impl(const uint8_t *chunk, size_t n, size_t slice_begin, si
     a.deferred_cap = deferred_capacity(n);
     a.deferred = (uint64_t *)workspace + ws_lookback_words((size_t)n_tiles_total);
     a.lut = lut256; a.k = k; a.window = window; a.n_bins = (uint64_t)n_bins; a.hist = (unsigned long long *)hist;
+    a.canon_xor = canon_xor;
     if (slice_begin == 0) {
         BNPK_CUDA(cudaMemsetAsync(workspace, 0, ws_lookback_words((size_t)n_tiles_total) * sizeof(uint64_t), st));
         cr_detect_kernel<<<1, 32, 0, st>>>(chunk, std::min(n, slice_end), lpe, trim_cr, status);
@@ -591,7 +612,7 @@ int chunk_kmer_count_impl(const uint8_t *chunk, size_t n, size_t slice_begin, si
     const bool smem_hist = use_smem_hist(n_bins, hist_mode);
     // tables between 32 MiB and 128 MiB of int64: count in the 32-bit scratch (a bin cannot overflow: n < 2^32 bytes)
     const bool scratch32 = !smem_hist && n_bins > (1ll << 22) && n_bins <= kScratch32MaxBins && n < (1ull << 32) &&
-                           tma_kernel_allowed() && tma_count_eligible(a, smem_hist);
+                           count_takes_scratch32(a, smem_hist);
     if (scratch32) {
         a.hist32 = reinterpret_cast<uint32_t *>(reinterpret_cast<uint8_t *>(workspace) + ws_core_bytes(n));
         if (slice_begin == 0) BNPK_CUDA(cudaMemsetAsync(a.hist32, 0, (size_t)n_bins * sizeof(uint32_t), st));
@@ -606,7 +627,7 @@ int chunk_kmer_count_impl(const uint8_t *chunk, size_t n, size_t slice_begin, si
         finalize_status_kernel<<<1, 32, 0, st>>>(status, lpe);
         BNPK_LAUNCHED("finalize_status_kernel");
         rc = count_fixups_impl(chunk, n, lpe, enc_mode, lut256, k, window, n_bins, hist, status,
-                               (uint64_t *)workspace + kWsDeferred, a.deferred, a.deferred_cap, st);
+                               (uint64_t *)workspace + kWsDeferred, a.deferred, a.deferred_cap, st, canon_xor);
     }
     return rc;
 }

@@ -128,16 +128,27 @@ class CudaOneLineBuffer:
     def can_fuse_count(self) -> bool:
         return True
 
-    def fused_kmer_histogram(self, k, window_size, n_bins, enc_mode, lut):
-        hist, status = ops.chunk_kmer_count(self._data, k, n_bins, None, window_size, self.n_lines_per_entry,
-                                            ord(self.HEADER), False, 1 if self._cr else 0, enc_mode, lut)
+    def fused_kmer_histogram(self, k, window_size, n_bins, enc_mode, lut, complement_xor=0):
+        """Histogram of the k-mers (window_size = 0) or minimizers of the sequence lines; complement_xor != 0 counts
+        canonical k-mers (min of a k-mer and its reverse complement) instead."""
+        if complement_xor:
+            assert window_size == 0, "canonical minimizers are not implemented"
+            hist, status = ops.chunk_kmer_count_canonical(self._data, k, complement_xor, n_bins, None, self.n_lines_per_entry,
+                                                          ord(self.HEADER), False, 1 if self._cr else 0, enc_mode, lut)
+        else:
+            hist, status = ops.chunk_kmer_count(self._data, k, n_bins, None, window_size, self.n_lines_per_entry,
+                                                ord(self.HEADER), False, 1 if self._cr else 0, enc_mode, lut)
         st = ops.read_status(status)
         if st.overflow:
             # pathological line structure (more odd rows than the fused pass keeps scratch for):
             # take the general two-kernel route over the row-offset vector instead
             seq = self.get_field_by_number(1)
-            hist, status = ops.rows_kmer_count(seq._data, seq._starts.contiguous(), seq._lens.contiguous(), enc_mode,
-                                               k, n_bins, window_size, lut)
+            if complement_xor:
+                hist, status = ops.rows_kmer_count_canonical(seq._data, seq._starts.contiguous(), seq._lens.contiguous(),
+                                                             enc_mode, k, complement_xor, n_bins, lut)
+            else:
+                hist, status = ops.rows_kmer_count(seq._data, seq._starts.contiguous(), seq._lens.contiguous(), enc_mode,
+                                                   k, n_bins, window_size, lut)
             st = ops.read_status(status)
         bad = st.bad_base(self._n_records)
         if bad is not None:

@@ -124,6 +124,27 @@ def chunk_kmer_count(chunk, k, n_bins, hist=None, window_size=0, lines_per_entry
 
 
 @_on_device
+def chunk_kmer_count_canonical(chunk, k, complement_xor, n_bins, hist=None, lines_per_entry=4, header_char=ord("@"),
+                               check_plus=True, trim_cr=-1, enc_mode=nv.ENC_ASCII_ACGT, lut=None, hist_mode=nv.HIST_AUTO,
+                               status=None):
+    """EXTENSION: K6 on canonical k-mers, min(h, hash of the reverse complement), of a device-resident chunk.
+    ``complement_xor``: 3 for ACGT-ordered alphabets, 2 for ACTG.  Accumulates into ``hist`` (int64[n_bins]);
+    returns (hist, status tensor)."""
+    _need_cuda(chunk, "chunk")
+    n = chunk.numel()
+    dev = chunk.device
+    if hist is None:
+        hist = torch.zeros(n_bins, dtype=torch.int64, device=dev)
+    if status is None:
+        status = nv.new_status(dev)
+    ws = nv.workspace(n, dev)
+    check(lib().bnpk_chunk_kmer_count_canonical(ptr(chunk), n, 0, n, 1, lines_per_entry, header_char, int(check_plus),
+                                                trim_cr, enc_mode, ptr(lut), k, complement_xor, n_bins, hist_mode,
+                                                ptr(hist), ptr(status), ptr(ws), ws.numel(), stream_ptr()))
+    return hist, status
+
+
+@_on_device
 def row_offsets(lens, shrink=0):
     """int64[R+1] exclusive prefix sums of max(lens - shrink, 0)."""
     _need_cuda(lens, "lens")

@@ -155,13 +155,16 @@ class LazyKmerValues(EncodedRaggedArray):
         if s.alphabet_encoding.alphabet_size != 4:
             hist, _ = ops.bincount(self._data.contiguous(), n_bins)
             return hist
+        buf = s.chunk_buffer
+        if buf is not None and buf.can_fuse_count():
+            # an untouched sequence field of a file buffer: straight from the raw chunk bytes
+            if self._canonical:
+                return buf.fused_kmer_histogram(self._k, 0, n_bins, s.enc_mode, s.lut, complement_xor=self._cxor)
+            return buf.fused_kmer_histogram(self._k, self._window, n_bins, s.enc_mode, s.lut)
         if self._canonical:
             hist, status = ops.rows_kmer_count_canonical(s.base, s.starts, s.lens, s.enc_mode, self._k, self._cxor, n_bins, s.lut)
             self._check(status)
             return hist
-        buf = s.chunk_buffer
-        if buf is not None and buf.can_fuse_count():
-            return buf.fused_kmer_histogram(self._k, self._window, n_bins, s.enc_mode, s.lut)
         span = self._window if self._window else self._k
         p_starts, p_lens, _ = _split_long_rows(s.starts, s.lens, span)
         hist, status = ops.rows_kmer_count(s.base, p_starts, p_lens, s.enc_mode, self._k, n_bins, self._window, s.lut)

@@ -199,6 +199,15 @@ int bnpk_rows_kmer_hash_canonical(const uint8_t *base, size_t base_bytes, const 
 int bnpk_rows_kmer_count_canonical(const uint8_t *base, size_t base_bytes, const int64_t *starts, const int32_t *lens,
                                    size_t n_rows, int enc_mode, const uint8_t *lut256, int k, int complement_xor,
                                    int64_t n_bins, int hist_mode, int64_t *hist, int64_t *status, void *stream);
+/*     The K6 fused count of canonical k-mers straight from raw chunk bytes: the arguments of bnpk_chunk_kmer_count
+ *     with complement_xor in place of window_size (canonical minimizers are not implemented).  Counts the values
+ *     bnpk_rows_kmer_count_canonical counts over the sequence lines of the chunk's complete entries; slices, status and
+ *     workspace as for bnpk_chunk_kmer_count.  complement_xor outside 1..3 returns BNPK_E_BADARG before any CUDA call. */
+int bnpk_chunk_kmer_count_canonical(const uint8_t *chunk, size_t n, size_t slice_begin, size_t slice_end,
+                                    int final_slice, int lines_per_entry, uint8_t header_char, int check_plus,
+                                    int trim_cr, int enc_mode, const uint8_t *lut256, int k, int complement_xor,
+                                    int64_t n_bins, int hist_mode, int64_t *hist,
+                                    int64_t *status, void *workspace, size_t workspace_bytes, void *stream);
 
 /* K5  np.bincount(values % n_bins, minlength=n_bins) accumulated into hist
  *     (sequence/count_encoded.py:173-177; EncodedArray.__array_function__ encoded_array.py:459-460).
