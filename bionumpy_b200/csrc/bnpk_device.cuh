@@ -30,8 +30,27 @@ constexpr uint64_t kValueMask = (1ull << 62) - 1;
 // workspace header (uint64 words)
 constexpr int kWsTicket = 0;        // per-launch tile ticket
 constexpr int kWsDeferred = 1;      // number of deferred (long) rows
-constexpr int kWsCarry = 2;         // newlines in all tiles of the earlier launches (slices) of this chunk
+constexpr int kWsLines = 3;         // ws kernels: newlines of the whole chunk (resolve pass)
+// ws kernels: labels as tile-major keys until the resolve pass turns them into entry indices (words 4..11 hold the
+// development stage clocks, BNPK_WS_DEBUG).  key = tile << 14 | entry of the tile (the entry index counted from the
+// tile's first line: at most (3 + 16383 + 1) >> 1 < 2^14); BAD_BASE's key = tile << 24 | entry << 10 | position in
+// the row (rows counted in the tile are at most 1024 bytes).  Keys ordered by tile are ordered by line, so min / max
+// over keys pick the same record as over entry indices.
+constexpr int kWsKeyHeader = 12;    // min key of a bad header line (all ones: none)
+constexpr int kWsKeyPlus = 13;      // min key of a bad '+' line (all ones: none)
+constexpr int kWsKeyBase = 14;      // min BAD_BASE key (all ones: none)
+constexpr int kWsKeyLastRow = 15;   // 1 + max key of a tile's last counted row (0: none)
 constexpr int kWsHeaderWords = 16;
+constexpr int kKeyEntryBits = 14, kKeyPosBits = 10;
+// deferred-row entries of the ws kernels hold a key; this bit marks a row the resolve pass deferred from a tile whose
+// record phase was not fixed locally (it counts as a long row only if the in-tile walk would have deferred it too)
+constexpr uint64_t kDeferredResolved = 1ull << 62;
+// ws kernels: per-tile word in tile_state[] = newlines of the tile | record phase guessed from its bytes << 16 |
+// kTileWordAmbiguous when no single phase was left (a tile has at most 16384 newlines: 15 bits)
+constexpr int kTileWordPhaseShift = 16;
+constexpr uint64_t kTileWordAmbiguous = 1ull << 18;
+constexpr int kWsSlotBytes = kTileBytes + 512;   // ws kernels: tile + halo staged per ring slot
+constexpr int kWsRowMax = 1024;                  // ws kernels: longer rows take the deferred pass
 
 __device__ __forceinline__ uint64_t ld_relaxed(const uint64_t *p) {
     uint64_t v;

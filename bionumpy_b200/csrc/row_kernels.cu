@@ -174,12 +174,17 @@ __global__ void __launch_bounds__(kRowThreads) rows_kernel(const RowArgs a) {
         int64_t start, L, r, out_off = 0;
         if (DEFERRED) {
             start = (int64_t)a.deferred[2 * row];
-            r = (int64_t)a.deferred[2 * row + 1];
+            const uint64_t rw = a.deferred[2 * row + 1];
+            r = (int64_t)(rw & ~kDeferredResolved);
             if (r >= n_records) continue;                     // belongs to a trailing incomplete entry
             L = warp_line_len(a.base, a.base_bytes, start, lane);
             if (L < 0) continue;
+            const int64_t end = start + L;                    // its newline
             if (cr && L > 0 && a.base[start + L - 1] == '\r') L -= 1;
-            if (lane == 0) ++acc_long;
+            // a row of a tile the ws resolve pass walked is a long row only if the in-tile walk would have deferred it:
+            // its newline past the tile's slot, or more than kWsRowMax bytes
+            const int64_t slot_end = ((start - 1) & ~(int64_t)(kTileBytes - 1)) + kWsSlotBytes;
+            if (lane == 0 && (!(rw & kDeferredResolved) || end >= slot_end || L > kWsRowMax)) ++acc_long;
         } else {
             start = a.starts[row];
             L = a.lens[row];

@@ -193,5 +193,7 @@ bool wsm_count_eligible(const TileArgs &a, bool smem_hist);
 int launch_wsm_count(const TileArgs &a, int enc_mode, bool smem_hist, cudaStream_t st);
 bool wsc_count_eligible(const TileArgs &a, bool smem_hist);
 int launch_wsc_count(const TileArgs &a, int enc_mode, bool smem_hist, cudaStream_t st);
+// after the last launch of a chunk through one of the ws builds: line prefix, phase check, keys -> entry indices
+int ws_resolve(const TileArgs &a, cudaStream_t st);
 
 }  // namespace bnpk

@@ -525,18 +525,25 @@ static bool count_takes_scratch32(const TileArgs &a, bool smem_hist) {
     return tma_kernel_allowed() && tma_count_eligible(a, smem_hist);
 }
 
-static int launch_count(const TileArgs &a, int enc_mode, bool smem_hist, cudaStream_t st) {
+// *ws_labels: the launch went to one of the ws builds, whose labels the resolve pass (ws_resolve) completes
+static int launch_count(const TileArgs &a, int enc_mode, bool smem_hist, cudaStream_t st, bool *ws_labels) {
+    *ws_labels = false;
     if (a.canon_xor) {
         // canonical k-mers: the wsc build for CTA-private tables of up to 2^14 bins, the register-staged kernel for the
         // rest (the round-1 kernel has no canonical build)
-        if (tma_kernel_allowed() && wsc_count_eligible(a, smem_hist)) return launch_wsc_count(a, enc_mode, smem_hist, st);
+        if (tma_kernel_allowed() && wsc_count_eligible(a, smem_hist)) {
+            *ws_labels = true;
+            return launch_wsc_count(a, enc_mode, smem_hist, st);
+        }
     } else if (tma_kernel_allowed() && tile_kernel_choice() != 1 && wsm_count_eligible(a, smem_hist)) {
+        *ws_labels = true;
         return launch_wsm_count(a, enc_mode, smem_hist, st);          // minimizers, windows of up to 12 k-mers
     } else if (tma_kernel_allowed() && tma_count_eligible(a, smem_hist)) {
         // the warp-specialised kernel for CTA-private tables; global tables are bound by L2 atomics, where the round-1
         // kernel's 21 row warps per SM keep more of them in flight (2^24 bins: 6.6 ms against 9.3 ms)
-        return (tile_kernel_choice() == 1 || (!smem_hist && tile_kernel_choice() != 3)) ? launch_tma_count(a, enc_mode, smem_hist, st)
-                                                                                       : launch_ws_count(a, enc_mode, smem_hist, st);
+        if (tile_kernel_choice() == 1 || (!smem_hist && tile_kernel_choice() != 3)) return launch_tma_count(a, enc_mode, smem_hist, st);
+        *ws_labels = true;
+        return launch_ws_count(a, enc_mode, smem_hist, st);
     }
     switch (enc_mode) {
         case BNPK_ENC_ASCII_ACGT: return launch_count_enc<BNPK_ENC_ASCII_ACGT>(a, smem_hist, st);
@@ -605,6 +612,8 @@ int chunk_kmer_count_impl(const uint8_t *chunk, size_t n, size_t slice_begin, si
     a.canon_xor = canon_xor;
     if (slice_begin == 0) {
         BNPK_CUDA(cudaMemsetAsync(workspace, 0, ws_lookback_words((size_t)n_tiles_total) * sizeof(uint64_t), st));
+        // the ws builds' min-keys start at "none" (all ones)
+        BNPK_CUDA(cudaMemsetAsync(a.ws + kWsKeyHeader, 0xFF, (kWsKeyBase - kWsKeyHeader + 1) * sizeof(uint64_t), st));
         cr_detect_kernel<<<1, 32, 0, st>>>(chunk, std::min(n, slice_end), lpe, trim_cr, status);
         BNPK_LAUNCHED("cr_detect_kernel");
     }
@@ -617,13 +626,15 @@ int chunk_kmer_count_impl(const uint8_t *chunk, size_t n, size_t slice_begin, si
         a.hist32 = reinterpret_cast<uint32_t *>(reinterpret_cast<uint8_t *>(workspace) + ws_core_bytes(n));
         if (slice_begin == 0) BNPK_CUDA(cudaMemsetAsync(a.hist32, 0, (size_t)n_bins * sizeof(uint32_t), st));
     }
-    int rc = launch_count(a, enc_mode, smem_hist, st);
+    bool ws_labels = false;
+    int rc = launch_count(a, enc_mode, smem_hist, st, &ws_labels);
     if (rc) return rc;
     if (final_slice && scratch32) {
         widen_add_kernel<<<sm_count() * 8, 256, 0, st>>>(a.hist32, a.hist, (size_t)n_bins);
         BNPK_LAUNCHED("widen_add_kernel");
     }
     if (final_slice) {
+        if (ws_labels && (rc = ws_resolve(a, st))) return rc;
         finalize_status_kernel<<<1, 32, 0, st>>>(status, lpe);
         BNPK_LAUNCHED("finalize_status_kernel");
         rc = count_fixups_impl(chunk, n, lpe, enc_mode, lut256, k, window, n_bins, hist, status,

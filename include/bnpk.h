@@ -72,7 +72,9 @@ enum {
     BNPK_ST_CR = 9,            /* 1 if '\r' trimming is active (io/one_line_buffer.py:175-182) */
     BNPK_ST_LAST_ROW_START = 10, /* internal: 1 + start of the last sequence line counted  */
     BNPK_ST_LAST_ROW_INDEX = 11, /* internal: 1 + its entry index                          */
-    BNPK_ST_OVERFLOW = 12,     /* != 0: the fused pass met more long/odd rows than its scratch holds;
+    BNPK_ST_OVERFLOW = 12,     /* != 0: the fused pass met more long/odd rows than its scratch holds,
+                                  or (malformed input) the record phase it read from a tile's own
+                                  bytes was not the one the line count gives;
                                   the counts are incomplete -- use bnpk_line_split + bnpk_rows_kmer_count */
     BNPK_ST_WORDS = 16
 };

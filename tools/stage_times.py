@@ -15,5 +15,5 @@ a.record(); ops.chunk_kmer_count(chunk, 31, 1 << 14, hist=hist, status=status); 
 w = ws.view(torch.int64)[:16].cpu().tolist()
 tiles, chunks = max(w[10], 1), max(w[11], 1)
 f = 1.0 / 1.965e3   # cycles -> us at 1965 MHz
-print("ms %.3f | per tile (us): copy %.2f  scan %.2f  lookback %.2f | per chunk: queue wait %.2f  chunk %.2f | P waits for a free slot %.2f us per tile | tiles %d chunks %d" % (
+print("ms %.3f | per tile (us): copy %.2f  scan %.2f  phase check + push %.2f | per chunk: queue wait %.2f  chunk %.2f | P waits for a free slot %.2f us per tile | tiles %d chunks %d" % (
     a.elapsed_time(b), w[4] / tiles * f, w[5] / tiles * f, w[6] / tiles * f, w[7] / chunks * f, w[8] / chunks * f, w[9] / tiles * f, tiles, chunks))
