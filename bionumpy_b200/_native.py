@@ -51,6 +51,11 @@ SIGNATURES = {
     "bnpk_rows_reverse_complement": (_i, [_vp, _sz, _vp, _vp, _sz, _vp, _vp, _vp, _vp]),
     "bnpk_rows_kmer_hash_canonical": (_i, [_vp, _sz, _vp, _vp, _sz, _i, _vp, _i, _i, _vp, _vp, _vp, _vp]),
     "bnpk_rows_kmer_count_canonical": (_i, [_vp, _sz, _vp, _vp, _sz, _i, _vp, _i, _i, _i64, _i, _vp, _vp, _vp]),
+    "bnpk_rows_minimizers_canonical": (_i, [_vp, _sz, _vp, _vp, _sz, _i, _vp, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "bnpk_rows_minimizer_count_canonical": (_i, [_vp, _sz, _vp, _vp, _sz, _i, _vp, _i, _i, _i, _i64, _i, _vp, _vp,
+                                                 _vp]),
+    "bnpk_chunk_minimizer_count_canonical": (_i, [_vp, _sz, _sz, _sz, _i, _i, _u8, _i, _i, _i, _vp, _i, _i, _i, _i64,
+                                                  _i, _vp, _vp, _vp, _sz, _vp]),
     "bnpk_bincount": (_i, [_vp, _sz, _i64, _i, _vp, _vp, _vp]),
     "bnpk_bincount_rows": (_i, [_vp, _vp, _sz, _i64, _vp, _vp, _vp]),
     "bnpk_pipeline_create": (_i, [ctypes.POINTER(_vp), _sz, _sz]),

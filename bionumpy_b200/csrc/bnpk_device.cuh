@@ -365,6 +365,7 @@ __device__ __forceinline__ uint32_t row_count(const uint32_t *s_codes, int b0, i
             }
         }
     } else {
+        // canon_xor != 0: canonical minimizers, the minimum of the canonical hashes of the window
         const int w = window - k + 1;           // k-mers per window (minimizers.py:52)
         const int nout = L - window + 1;        // windows in the row
         const int nh = L - k + 1;               // hashes in the row
@@ -372,8 +373,11 @@ __device__ __forceinline__ uint32_t row_count(const uint32_t *s_codes, int b0, i
             const int step = 32 - (w - 1);
             for (int base = 0; base < nout; base += step) {
                 const int p = base + lane;
-                uint64_t h = ~0ull;
-                if (p < nh) h = stream_64(s_codes, (uint32_t)(b0 + p)) & kmask;
+                uint64_t h = ~0ull;             // lanes past the last hash keep the sentinel
+                if (p < nh) {
+                    h = stream_64(s_codes, (uint32_t)(b0 + p)) & kmask;
+                    if (ht.canon_xor) h = canonical_hash(h, k, ht.canon_xor);
+                }
                 const uint64_t m = warp_sliding_min(h, w);
                 if (lane < step && p < nout) { hist_add<SMEM_HIST>(ht, m); ++produced; }
             }
@@ -381,7 +385,8 @@ __device__ __forceinline__ uint32_t row_count(const uint32_t *s_codes, int b0, i
             for (int j = lane; j < nout; j += 32) {
                 uint64_t m = ~0ull;
                 for (int i = 0; i < w; ++i) {
-                    const uint64_t h = stream_64(s_codes, (uint32_t)(b0 + j + i)) & kmask;
+                    uint64_t h = stream_64(s_codes, (uint32_t)(b0 + j + i)) & kmask;
+                    if (ht.canon_xor) h = canonical_hash(h, k, ht.canon_xor);
                     m = h < m ? h : m;
                 }
                 hist_add<SMEM_HIST>(ht, m);

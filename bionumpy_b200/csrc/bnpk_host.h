@@ -45,7 +45,7 @@ inline uint64_t canon_pattern(int complement_xor) {
     return complement_xor == 3 ? ~0ull : complement_xor == 2 ? 0xAAAAAAAAAAAAAAAAull : 0x5555555555555555ull;
 }
 
-// canon_xor != 0: count canonical k-mers (window must be 0)
+// canon_xor != 0: count canonical k-mers (window 0) or canonical minimizers (window > 0)
 int chunk_kmer_count_impl(const uint8_t *chunk, size_t n, size_t slice_begin, size_t slice_end, int final_slice,
                           int lpe, uint8_t header_char, int check_plus, int trim_cr, int enc_mode,
                           const uint8_t *lut256, int k, int window, int64_t n_bins, int hist_mode, int64_t *hist,

@@ -422,6 +422,18 @@ int bnpk_chunk_kmer_count_canonical(const uint8_t *chunk, size_t n, size_t slice
                                  workspace, workspace_bytes, (cudaStream_t)stream, canon_pattern(complement_xor));
 }
 
+int bnpk_chunk_minimizer_count_canonical(const uint8_t *chunk, size_t n, size_t slice_begin, size_t slice_end,
+                                         int final_slice, int lines_per_entry, uint8_t header_char, int check_plus,
+                                         int trim_cr, int enc_mode, const uint8_t *lut256, int k, int window_size,
+                                         int complement_xor, int64_t n_bins, int hist_mode, int64_t *hist,
+                                         int64_t *status, void *workspace, size_t workspace_bytes, void *stream) {
+    if (complement_xor < 1 || complement_xor > 3) return set_err(BNPK_E_BADARG, "complement_xor must be 1, 2 or 3");
+    if (window_size < 1) return set_err(BNPK_E_WINDOW, "window_size must be positive");
+    return chunk_kmer_count_impl(chunk, n, slice_begin, slice_end, final_slice, lines_per_entry, header_char,
+                                 check_plus, trim_cr, enc_mode, lut256, k, window_size, n_bins, hist_mode, hist, status,
+                                 workspace, workspace_bytes, (cudaStream_t)stream, canon_pattern(complement_xor));
+}
+
 int bnpk_row_offsets(const int32_t *lens, size_t n_rows, int shrink, int64_t *offsets, void *workspace,
                      size_t workspace_bytes, void *stream) {
     cudaStream_t st = (cudaStream_t)stream;

@@ -37,7 +37,7 @@ struct RowArgs {
     const uint64_t *deferred;
     size_t deferred_cap;
     int lpe;
-    uint64_t canon_xor;          // != 0: canonical k-mers (hash / count modes without a minimizer window)
+    uint64_t canon_xor;          // != 0: canonical k-mers, or canonical minimizers with a window
 };
 
 template <int RM, int ENC, bool SMEM_HIST>
@@ -114,8 +114,11 @@ __device__ void warp_row(const RowArgs &a, uint32_t *w_codes, uint32_t *w_flags,
                 const int step = 32 - (w - 1);
                 for (int base = 0; base < nout; base += step) {
                     const int p = base + lane;
-                    uint64_t h = ~0ull;
-                    if (p < nh) h = stream_64(w_codes, (uint32_t)(off + p)) & kmask;
+                    uint64_t h = ~0ull;                       // lanes past the last hash keep the sentinel
+                    if (p < nh) {
+                        h = stream_64(w_codes, (uint32_t)(off + p)) & kmask;
+                        if (a.canon_xor) h = canonical_hash(h, a.k, a.canon_xor);
+                    }
                     const uint64_t m = warp_sliding_min(h, w);
                     if (lane < step && p < nout) { out[p] = (int64_t)m; ++acc_values; }
                 }
@@ -123,7 +126,8 @@ __device__ void warp_row(const RowArgs &a, uint32_t *w_codes, uint32_t *w_flags,
                 for (int j = lane; j < nout; j += 32) {
                     uint64_t m = ~0ull;
                     for (int i = 0; i < w; ++i) {
-                        const uint64_t h = stream_64(w_codes, (uint32_t)(off + j + i)) & kmask;
+                        uint64_t h = stream_64(w_codes, (uint32_t)(off + j + i)) & kmask;
+                        if (a.canon_xor) h = canonical_hash(h, a.k, a.canon_xor);
                         m = h < m ? h : m;
                     }
                     out[j] = (int64_t)m;
@@ -480,6 +484,40 @@ int bnpk_rows_kmer_count_canonical(const uint8_t *base, size_t base_bytes, const
     cudaStream_t st = (cudaStream_t)stream;
     return use_smem_hist(n_bins, hist_mode) ? launch_rows_enc<RM_COUNT, true, false>(a, enc_mode, n_rows, st)
                                             : launch_rows_enc<RM_COUNT, false, false>(a, enc_mode, n_rows, st);
+}
+
+int bnpk_rows_minimizers_canonical(const uint8_t *base, size_t base_bytes, const int64_t *starts, const int32_t *lens,
+                                   size_t n_rows, int enc_mode, const uint8_t *lut256, int k, int window_size,
+                                   int complement_xor, const int64_t *offsets, int64_t *mins_out, int64_t *status,
+                                   void *stream) {
+    if (complement_xor < 1 || complement_xor > 3) return set_err(BNPK_E_BADARG, "complement_xor must be 1, 2 or 3");
+    if (window_size < 1) return set_err(BNPK_E_WINDOW, "window_size must be positive");
+    if (int rc = check_common(enc_mode, lut256, k, window_size)) return rc;
+    if (n_rows == 0) return 0;
+    RowArgs a{};
+    a.base = base; a.base_bytes = base_bytes; a.starts = starts; a.lens = lens; a.n_rows = n_rows; a.lut = lut256;
+    a.k = k; a.window = window_size; a.offsets = offsets; a.out = mins_out; a.n_bins = 1; a.status = status;
+    a.canon_xor = canon_pattern(complement_xor);
+    return launch_rows_enc<RM_MINIMIZER, false, false>(a, enc_mode, n_rows, (cudaStream_t)stream);
+}
+
+int bnpk_rows_minimizer_count_canonical(const uint8_t *base, size_t base_bytes, const int64_t *starts,
+                                        const int32_t *lens, size_t n_rows, int enc_mode, const uint8_t *lut256, int k,
+                                        int window_size, int complement_xor, int64_t n_bins, int hist_mode,
+                                        int64_t *hist, int64_t *status, void *stream) {
+    if (complement_xor < 1 || complement_xor > 3) return set_err(BNPK_E_BADARG, "complement_xor must be 1, 2 or 3");
+    if (window_size < 1) return set_err(BNPK_E_WINDOW, "window_size must be positive");
+    if (int rc = check_common(enc_mode, lut256, k, window_size)) return rc;
+    if (n_bins < 1) return set_err(BNPK_E_BINS, "n_bins must be positive");
+    if (hist_mode == BNPK_HIST_SMEM && n_bins > kSmemMaxBins) return set_err(BNPK_E_BINS, "too many bins for the shared-memory histogram");
+    if (n_rows == 0) return 0;
+    RowArgs a{};
+    a.base = base; a.base_bytes = base_bytes; a.starts = starts; a.lens = lens; a.n_rows = n_rows; a.lut = lut256;
+    a.k = k; a.window = window_size; a.n_bins = (uint64_t)n_bins; a.hist = (unsigned long long *)hist; a.status = status;
+    a.canon_xor = canon_pattern(complement_xor);
+    cudaStream_t st = (cudaStream_t)stream;
+    return use_smem_hist(n_bins, hist_mode) ? launch_rows_enc<RM_COUNT_MIN, true, false>(a, enc_mode, n_rows, st)
+                                            : launch_rows_enc<RM_COUNT_MIN, false, false>(a, enc_mode, n_rows, st);
 }
 
 int bnpk_rows_reverse_complement(const uint8_t *base, size_t base_bytes, const int64_t *starts, const int32_t *lens,

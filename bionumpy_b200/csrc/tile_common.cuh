@@ -28,7 +28,7 @@ struct TileArgs {
     uint64_t n_bins;
     unsigned long long *hist;
     uint32_t *hist32;              // optional 32-bit scratch table in the workspace (large global tables), else null
-    uint64_t canon_xor;            // != 0: canonical k-mers, the complement as an XOR pattern (canon_pattern)
+    uint64_t canon_xor;            // != 0: canonical k-mers / minimizers, the complement as an XOR pattern (canon_pattern)
 };
 
 // 256-bit streaming load (sm_100: LDG.E.256), read-only path, no L1 allocation
@@ -193,6 +193,7 @@ bool wsm_count_eligible(const TileArgs &a, bool smem_hist);
 int launch_wsm_count(const TileArgs &a, int enc_mode, bool smem_hist, cudaStream_t st);
 bool wsc_count_eligible(const TileArgs &a, bool smem_hist);
 int launch_wsc_count(const TileArgs &a, int enc_mode, bool smem_hist, cudaStream_t st);
+int launch_wsmc_count(const TileArgs &a, int enc_mode, bool smem_hist, cudaStream_t st);   // canonical minimizers, wsm_count_eligible
 // after the last launch of a chunk through one of the ws builds: line prefix, phase check, keys -> entry indices
 int ws_resolve(const TileArgs &a, cudaStream_t st);
 

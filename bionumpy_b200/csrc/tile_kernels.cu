@@ -519,16 +519,24 @@ static int tile_kernel_choice() {
 static bool tma_kernel_allowed() { return tile_kernel_choice() != 0; }
 
 // the kernel a fused count of a global table goes to writes the 32-bit scratch table (a.hist32) when it gets one: the
-// tma / ws kernels, and for canonical k-mers tile_kernel (global canonical tables always go there)
+// tma / ws kernels, and for canonical k-mers tile_kernel (global canonical tables always go there).  The minimizer
+// walk of tile_kernel (row_count) counts into the int64 table, so canonical minimizers get no scratch.
 static bool count_takes_scratch32(const TileArgs &a, bool smem_hist) {
-    if (a.canon_xor) return !smem_hist;
+    if (a.canon_xor) return !smem_hist && a.window == 0;
     return tma_kernel_allowed() && tma_count_eligible(a, smem_hist);
 }
 
 // *ws_labels: the launch went to one of the ws builds, whose labels the resolve pass (ws_resolve) completes
 static int launch_count(const TileArgs &a, int enc_mode, bool smem_hist, cudaStream_t st, bool *ws_labels) {
     *ws_labels = false;
-    if (a.canon_xor) {
+    if (a.canon_xor && a.window) {
+        // canonical minimizers: the wsmc build where wsm would take the count (CTA-private table of up to 2^14 bins,
+        // windows of up to 12 k-mers), the register-staged kernel for the rest
+        if (tma_kernel_allowed() && tile_kernel_choice() != 1 && wsm_count_eligible(a, smem_hist)) {
+            *ws_labels = true;
+            return launch_wsmc_count(a, enc_mode, smem_hist, st);
+        }
+    } else if (a.canon_xor) {
         // canonical k-mers: the wsc build for CTA-private tables of up to 2^14 bins, the register-staged kernel for the
         // rest (the round-1 kernel has no canonical build)
         if (tma_kernel_allowed() && wsc_count_eligible(a, smem_hist)) {
@@ -583,7 +591,6 @@ int chunk_kmer_count_impl(const uint8_t *chunk, size_t n, size_t slice_begin, si
                           const uint8_t *lut256, int k, int window, int64_t n_bins, int hist_mode, int64_t *hist,
                           int64_t *status, void *workspace, size_t workspace_bytes, cudaStream_t st, uint64_t canon_xor) {
     if (k < 1 || k > 31) return set_err(BNPK_E_K, "k must be larger than 0 and smaller than 32");
-    if (canon_xor != 0 && window != 0) return set_err(BNPK_E_BADARG, "canonical minimizers are not implemented");
     if (window != 0 && window < k) return set_err(BNPK_E_WINDOW, "kmer size must be smaller than window size");
     if (window > 1024) return set_err(BNPK_E_WINDOW, "window_size above 1024 is not supported");
     if (n_bins < 1) return set_err(BNPK_E_BINS, "n_bins must be positive");

@@ -1,4 +1,4 @@
-// tile_ws_kernel.cu -- the three builds of the warp-specialised fused count (tile_ws_kernel.inl)
+// tile_ws_kernel.cu -- the four builds of the warp-specialised fused count (tile_ws_kernel.inl)
 #include "tile_common.cuh"
 
 // k-mer counts: the dominant kernel of the hot path
@@ -44,10 +44,28 @@
 #define BNPK_WS_CANON 1
 #define BNPK_WS_LAUNCH launch_wsc_count
 #include "tile_ws_kernel.inl"
+#undef BNPK_WS_NAMESPACE
+#undef BNPK_WS_NS
+#undef BNPK_WS_SG
+#undef BNPK_WS_RW
+#undef BNPK_WS_MINZ
+#undef BNPK_WS_CANON
+#undef BNPK_WS_LAUNCH
+
+// canonical minimizer counts (the minimum of min(k-mer, reverse complement) over each window); the ring, geometry and
+// staging of the minimizer build
+#define BNPK_WS_NAMESPACE wsmc
+#define BNPK_WS_NS 4
+#define BNPK_WS_SG 1
+#define BNPK_WS_RW 14      // the reverse-complement words do not fit 80 registers (16 row warps: spills); 20 warps: 96, no stack
+#define BNPK_WS_MINZ 1
+#define BNPK_WS_CANON 1
+#define BNPK_WS_LAUNCH launch_wsmc_count
+#include "tile_ws_kernel.inl"
 
 namespace bnpk {
-// minimizer counts the wsm build takes: CTA-private table, windows of at most kMinzW k-mers; the rest (and global
-// tables) stay with the register-staged kernel
+// minimizer counts the wsm build (and, canonical, the wsmc build) takes: CTA-private table, windows of at most kMinzW
+// k-mers; the rest (and global tables) stay with the register-staged kernel
 bool wsm_count_eligible(const TileArgs &a, bool smem_hist) {
     if (a.window == 0 || !smem_hist || a.n_bins > (uint64_t)wsm::kMaxBins) return false;
     if (a.window - a.k + 1 > wsm::kMinzW) return false;
@@ -67,7 +85,7 @@ bool wsc_count_eligible(const TileArgs &a, bool smem_hist) {
 }
 }  // namespace bnpk
 
-// ---- resolve pass: after the last launch of a chunk through the ws / wsm / wsc builds ----------------------------------
+// ---- resolve pass: after the last launch of a chunk through the ws / wsm / wsc / wsmc builds -----------------------------
 // The kernel labels entries by tile-major keys and fixes each tile's record phase from the tile's own bytes.  Here the
 // tiles' newline counts are scanned (two-level: sums of 1024 tiles, then one block per 1024 tiles), every guessed phase
 // is checked against the line prefix (a wrong guess means the true phase breaks a line rule inside that tile: malformed

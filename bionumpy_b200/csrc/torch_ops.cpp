@@ -76,6 +76,29 @@ Tensor chunk_kmer_count_canonical(const Tensor &chunk, int64_t k, int64_t comple
     return status;
 }
 
+// K6 on canonical minimizers (min over each window of min(k-mer, reverse complement)): accumulated into hist.  Returns
+// the status block.
+Tensor chunk_minimizer_count_canonical(const Tensor &chunk, int64_t k, int64_t window_size, int64_t complement_xor,
+                                       Tensor hist, int64_t lines_per_entry, int64_t header_char, bool check_plus,
+                                       int64_t trim_cr, int64_t enc_mode, const c10::optional<Tensor> &lut,
+                                       int64_t hist_mode) {
+    need(chunk, torch::kUInt8, "chunk");
+    need(hist, torch::kInt64, "hist");
+    TORCH_CHECK(hist.get_device() == chunk.get_device(), "bnpk: chunk and hist on different devices");
+    c10::cuda::CUDAGuard guard(chunk.device());
+    Tensor status = new_status(chunk);
+    const size_t n = (size_t)chunk.numel();
+    Tensor ws = new_workspace(chunk, n);
+    check(bnpk_chunk_minimizer_count_canonical(chunk.data_ptr<uint8_t>(), n, 0, n, 1, (int)lines_per_entry,
+                                               (uint8_t)header_char, check_plus, (int)trim_cr, (int)enc_mode,
+                                               lut ? u8(*lut) : nullptr, (int)k, (int)window_size, (int)complement_xor,
+                                               hist.numel(), (int)hist_mode, hist.data_ptr<int64_t>(),
+                                               status.data_ptr<int64_t>(), ws.data_ptr<uint8_t>(), (size_t)ws.numel(),
+                                               cur_stream(chunk)),
+          "chunk_minimizer_count_canonical");
+    return status;
+}
+
 // K1: (starts int64[max_rows], lens int32[max_rows], status)
 std::tuple<Tensor, Tensor, Tensor> line_split(const Tensor &chunk, int64_t lines_per_entry, int64_t field_line,
                                               int64_t start_offset, int64_t header_char, bool check_plus,
@@ -137,7 +160,12 @@ std::tuple<Tensor, Tensor> rows_kmer_hash(const Tensor &base, const Tensor &star
     Tensor status = new_status(base);
     const uint8_t *l = lut ? u8(*lut) : nullptr;
     int rc;
-    if (window_size)
+    if (window_size && complement_xor)
+        rc = bnpk_rows_minimizers_canonical(base.data_ptr<uint8_t>(), (size_t)base.numel(), starts.data_ptr<int64_t>(),
+                                            lens.data_ptr<int32_t>(), (size_t)lens.numel(), (int)enc_mode, l, (int)k,
+                                            (int)window_size, (int)complement_xor, offsets.data_ptr<int64_t>(),
+                                            out.data_ptr<int64_t>(), status.data_ptr<int64_t>(), cur_stream(base));
+    else if (window_size)
         rc = bnpk_rows_minimizers(base.data_ptr<uint8_t>(), (size_t)base.numel(), starts.data_ptr<int64_t>(), lens.data_ptr<int32_t>(),
                                   (size_t)lens.numel(), (int)enc_mode, l, (int)k, (int)window_size, offsets.data_ptr<int64_t>(),
                                   out.data_ptr<int64_t>(), status.data_ptr<int64_t>(), cur_stream(base));
@@ -164,7 +192,12 @@ Tensor rows_kmer_count(const Tensor &base, const Tensor &starts, const Tensor &l
     Tensor status = new_status(base);
     const uint8_t *l = lut ? u8(*lut) : nullptr;
     int rc;
-    if (complement_xor)
+    if (window_size && complement_xor)
+        rc = bnpk_rows_minimizer_count_canonical(base.data_ptr<uint8_t>(), (size_t)base.numel(), starts.data_ptr<int64_t>(),
+                                                 lens.data_ptr<int32_t>(), (size_t)lens.numel(), (int)enc_mode, l, (int)k,
+                                                 (int)window_size, (int)complement_xor, hist.numel(), (int)hist_mode,
+                                                 hist.data_ptr<int64_t>(), status.data_ptr<int64_t>(), cur_stream(base));
+    else if (complement_xor)
         rc = bnpk_rows_kmer_count_canonical(base.data_ptr<uint8_t>(), (size_t)base.numel(), starts.data_ptr<int64_t>(),
                                             lens.data_ptr<int32_t>(), (size_t)lens.numel(), (int)enc_mode, l, (int)k,
                                             (int)complement_xor, hist.numel(), (int)hist_mode, hist.data_ptr<int64_t>(),
@@ -211,6 +244,9 @@ TORCH_LIBRARY(bnpk, m) {
     m.def("chunk_kmer_count_canonical(Tensor chunk, int k, int complement_xor, Tensor(a!) hist, int lines_per_entry=4, "
           "int header_char=64, bool check_plus=True, int trim_cr=-1, int enc_mode=0, Tensor? lut=None, "
           "int hist_mode=0) -> Tensor");
+    m.def("chunk_minimizer_count_canonical(Tensor chunk, int k, int window_size, int complement_xor, Tensor(a!) hist, "
+          "int lines_per_entry=4, int header_char=64, bool check_plus=True, int trim_cr=-1, int enc_mode=0, "
+          "Tensor? lut=None, int hist_mode=0) -> Tensor");
     m.def("line_split(Tensor chunk, int lines_per_entry, int field_line, int start_offset, int header_char, "
           "bool check_plus, int trim_cr, int max_rows) -> (Tensor, Tensor, Tensor)");
     m.def("row_offsets(Tensor lens, int shrink) -> Tensor");
@@ -227,6 +263,7 @@ TORCH_LIBRARY(bnpk, m) {
 TORCH_LIBRARY_IMPL(bnpk, CUDA, m) {
     m.impl("chunk_kmer_count", &chunk_kmer_count);
     m.impl("chunk_kmer_count_canonical", &chunk_kmer_count_canonical);
+    m.impl("chunk_minimizer_count_canonical", &chunk_minimizer_count_canonical);
     m.impl("line_split", &line_split);
     m.impl("row_offsets", &row_offsets);
     m.impl("rows_encode", &rows_encode);

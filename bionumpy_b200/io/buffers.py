@@ -130,9 +130,12 @@ class CudaOneLineBuffer:
 
     def fused_kmer_histogram(self, k, window_size, n_bins, enc_mode, lut, complement_xor=0):
         """Histogram of the k-mers (window_size = 0) or minimizers of the sequence lines; complement_xor != 0 counts
-        canonical k-mers (min of a k-mer and its reverse complement) instead."""
-        if complement_xor:
-            assert window_size == 0, "canonical minimizers are not implemented"
+        canonical k-mers (min of a k-mer and its reverse complement) / canonical minimizers instead."""
+        if complement_xor and window_size:
+            hist, status = ops.chunk_minimizer_count_canonical(self._data, k, window_size, complement_xor, n_bins, None,
+                                                               self.n_lines_per_entry, ord(self.HEADER), False,
+                                                               1 if self._cr else 0, enc_mode, lut)
+        elif complement_xor:
             hist, status = ops.chunk_kmer_count_canonical(self._data, k, complement_xor, n_bins, None, self.n_lines_per_entry,
                                                           ord(self.HEADER), False, 1 if self._cr else 0, enc_mode, lut)
         else:
@@ -143,7 +146,11 @@ class CudaOneLineBuffer:
             # pathological line structure (more odd rows than the fused pass keeps scratch for):
             # take the general two-kernel route over the row-offset vector instead
             seq = self.get_field_by_number(1)
-            if complement_xor:
+            if complement_xor and window_size:
+                hist, status = ops.rows_minimizer_count_canonical(seq._data, seq._starts.contiguous(),
+                                                                  seq._lens.contiguous(), enc_mode, k, window_size,
+                                                                  complement_xor, n_bins, lut)
+            elif complement_xor:
                 hist, status = ops.rows_kmer_count_canonical(seq._data, seq._starts.contiguous(), seq._lens.contiguous(),
                                                              enc_mode, k, complement_xor, n_bins, lut)
             else:

@@ -145,6 +145,28 @@ def chunk_kmer_count_canonical(chunk, k, complement_xor, n_bins, hist=None, line
 
 
 @_on_device
+def chunk_minimizer_count_canonical(chunk, k, window_size, complement_xor, n_bins, hist=None, lines_per_entry=4,
+                                    header_char=ord("@"), check_plus=True, trim_cr=-1, enc_mode=nv.ENC_ASCII_ACGT,
+                                    lut=None, hist_mode=nv.HIST_AUTO, status=None):
+    """EXTENSION: K6 on canonical minimizers, the minimum over each window of ``window_size`` bases of
+    min(h, hash of the reverse complement), of a device-resident chunk.  ``complement_xor``: 3 for ACGT-ordered
+    alphabets, 2 for ACTG.  Accumulates into ``hist`` (int64[n_bins]); returns (hist, status tensor)."""
+    _need_cuda(chunk, "chunk")
+    n = chunk.numel()
+    dev = chunk.device
+    if hist is None:
+        hist = torch.zeros(n_bins, dtype=torch.int64, device=dev)
+    if status is None:
+        status = nv.new_status(dev)
+    ws = nv.workspace(n, dev)
+    check(lib().bnpk_chunk_minimizer_count_canonical(ptr(chunk), n, 0, n, 1, lines_per_entry, header_char,
+                                                     int(check_plus), trim_cr, enc_mode, ptr(lut), k, window_size,
+                                                     complement_xor, n_bins, hist_mode, ptr(hist), ptr(status), ptr(ws),
+                                                     ws.numel(), stream_ptr()))
+    return hist, status
+
+
+@_on_device
 def row_offsets(lens, shrink=0):
     """int64[R+1] exclusive prefix sums of max(lens - shrink, 0)."""
     _need_cuda(lens, "lens")
@@ -268,6 +290,36 @@ def rows_kmer_count_canonical(base, starts, lens, enc_mode, k, complement_xor, n
         status = nv.new_status(base.device)
     check(lib().bnpk_rows_kmer_count_canonical(*_rows_args(base, starts, lens), enc_mode, ptr(lut), k, complement_xor,
                                                n_bins, hist_mode, ptr(hist), ptr(status), stream_ptr()))
+    return hist, status
+
+
+@_on_device
+def rows_minimizers_canonical(base, starts, lens, enc_mode, k, window_size, complement_xor, lut=None, offsets=None,
+                              status=None, total=None):
+    """EXTENSION: canonical minimizers, the minimum over each window of min(h, hash of the reverse complement)
+    (K4 with a second strand)."""
+    if offsets is None:
+        offsets = row_offsets(lens, window_size - 1)
+    if total is None:
+        total = int(offsets[-1].item())
+    out = torch.empty(total, dtype=torch.int64, device=base.device)
+    if status is None:
+        status = nv.new_status(base.device)
+    check(lib().bnpk_rows_minimizers_canonical(*_rows_args(base, starts, lens), enc_mode, ptr(lut), k, window_size,
+                                               complement_xor, ptr(offsets), ptr(out), ptr(status), stream_ptr()))
+    return out, offsets, status
+
+
+@_on_device
+def rows_minimizer_count_canonical(base, starts, lens, enc_mode, k, window_size, complement_xor, n_bins, lut=None,
+                                   hist=None, hist_mode=nv.HIST_AUTO, status=None):
+    if hist is None:
+        hist = torch.zeros(n_bins, dtype=torch.int64, device=base.device)
+    if status is None:
+        status = nv.new_status(base.device)
+    check(lib().bnpk_rows_minimizer_count_canonical(*_rows_args(base, starts, lens), enc_mode, ptr(lut), k,
+                                                    window_size, complement_xor, n_bins, hist_mode, ptr(hist),
+                                                    ptr(status), stream_ptr()))
     return hist, status
 
 

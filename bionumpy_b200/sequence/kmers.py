@@ -84,7 +84,8 @@ class LazyKmerValues(EncodedRaggedArray):
         self._canonical = canonical
         if canonical:
             from .dna import complement_xor_of
-            assert window_size == 0, "canonical minimizers are not implemented"
+            if window_size and source.alphabet_encoding.alphabet_size != 4:
+                raise NotImplementedError("minimizers are only implemented for 4-letter alphabets")
             self._cxor = complement_xor_of(source.alphabet_encoding)
         shrink = (window_size if window_size else k) - 1
         self._lens = torch.clamp(source.lens - shrink, min=0).to(torch.int32)
@@ -116,7 +117,10 @@ class LazyKmerValues(EncodedRaggedArray):
                 p_off = torch.cat([p_off, offsets[-1:]]).contiguous()   # kernels read offsets[row] only
             else:
                 total, p_off = None, offsets
-            if self._window:
+            if self._window and self._canonical:
+                vals, _, status = ops.rows_minimizers_canonical(s.base, p_starts, p_lens, s.enc_mode, self._k,
+                                                                self._window, self._cxor, s.lut, p_off, total=total)
+            elif self._window:
                 vals, _, status = ops.rows_minimizers(s.base, p_starts, p_lens, s.enc_mode, self._k, self._window,
                                                       s.lut, p_off, total=total)
             elif self._canonical:
@@ -159,15 +163,21 @@ class LazyKmerValues(EncodedRaggedArray):
         if buf is not None and buf.can_fuse_count():
             # an untouched sequence field of a file buffer: straight from the raw chunk bytes
             if self._canonical:
-                return buf.fused_kmer_histogram(self._k, 0, n_bins, s.enc_mode, s.lut, complement_xor=self._cxor)
+                return buf.fused_kmer_histogram(self._k, self._window, n_bins, s.enc_mode, s.lut,
+                                                complement_xor=self._cxor)
             return buf.fused_kmer_histogram(self._k, self._window, n_bins, s.enc_mode, s.lut)
-        if self._canonical:
+        if self._canonical and not self._window:
             hist, status = ops.rows_kmer_count_canonical(s.base, s.starts, s.lens, s.enc_mode, self._k, self._cxor, n_bins, s.lut)
             self._check(status)
             return hist
         span = self._window if self._window else self._k
         p_starts, p_lens, _ = _split_long_rows(s.starts, s.lens, span)
-        hist, status = ops.rows_kmer_count(s.base, p_starts, p_lens, s.enc_mode, self._k, n_bins, self._window, s.lut)
+        if self._canonical:
+            hist, status = ops.rows_minimizer_count_canonical(s.base, p_starts, p_lens, s.enc_mode, self._k,
+                                                              self._window, self._cxor, n_bins, s.lut)
+        else:
+            hist, status = ops.rows_kmer_count(s.base, p_starts, p_lens, s.enc_mode, self._k, n_bins, self._window,
+                                               s.lut)
         self._check(status, split=p_starts is not s.starts)
         return hist
 
@@ -194,7 +204,7 @@ def count_kmers(sequence, k: int, axis=None) -> EncodedCounts:
 
 def count_kmers_hashed(sequence, k: int, n_buckets: int = 1 << 24, window_size: int = 0, canonical: bool = False) -> torch.Tensor:
     """EXTENSION: np.bincount(get_kmers(sequence, k) % n_buckets) (or of the minimizers when
-    window_size > 0) as an int64 CUDA tensor, fused."""
+    window_size > 0) as an int64 CUDA tensor, fused.  ``canonical=True`` counts canonical k-mers / minimizers."""
     assert 0 < k < 32, "k must be larger than 0 and smaller than 32"
     assert window_size == 0 or k <= window_size, "kmer size must be smaller than window size"
     return count_hashed(LazyKmerValues(_source_of(sequence), k, window_size, canonical=canonical), n_buckets)

@@ -7,13 +7,16 @@ from .kmers import LazyKmerValues, _source_of
 from .. import config
 
 
-def get_minimizers(sequence, k: int, window_size: int):
+def get_minimizers(sequence, k: int, window_size: int, canonical: bool = False):
+    """EXTENSION: ``canonical=True`` takes the minimum of min(hash, hash of the reverse complement) over each
+    window: a read and its reverse complement give the same values, window j of one being window
+    L - window_size - j of the other."""
     assert isinstance(sequence.encoding, AlphabetEncoding), \
         "Sequence needs to be encoded with an AlphabetEncoding, e.g. DNAEncoding"
     assert k <= window_size, "kmer size must be smaller than window size"
     assert 0 < k < 32, "k must be larger than 0 and smaller than 32"
     src = _source_of(sequence)
-    out = LazyKmerValues(src, k, window_size)
+    out = LazyKmerValues(src, k, window_size, canonical=canonical)
     if not config.LAZY:
         out._data
     if isinstance(sequence, EncodedArray):

@@ -202,14 +202,35 @@ int bnpk_rows_kmer_count_canonical(const uint8_t *base, size_t base_bytes, const
                                    size_t n_rows, int enc_mode, const uint8_t *lut256, int k, int complement_xor,
                                    int64_t n_bins, int hist_mode, int64_t *hist, int64_t *status, void *stream);
 /*     The K6 fused count of canonical k-mers straight from raw chunk bytes: the arguments of bnpk_chunk_kmer_count
- *     with complement_xor in place of window_size (canonical minimizers are not implemented).  Counts the values
- *     bnpk_rows_kmer_count_canonical counts over the sequence lines of the chunk's complete entries; slices, status and
- *     workspace as for bnpk_chunk_kmer_count.  complement_xor outside 1..3 returns BNPK_E_BADARG before any CUDA call. */
+ *     with complement_xor in place of window_size (canonical minimizers: bnpk_chunk_minimizer_count_canonical).  Counts
+ *     the values bnpk_rows_kmer_count_canonical counts over the sequence lines of the chunk's complete entries; slices,
+ *     status and workspace as for bnpk_chunk_kmer_count.  complement_xor outside 1..3 returns BNPK_E_BADARG before any
+ *     CUDA call. */
 int bnpk_chunk_kmer_count_canonical(const uint8_t *chunk, size_t n, size_t slice_begin, size_t slice_end,
                                     int final_slice, int lines_per_entry, uint8_t header_char, int check_plus,
                                     int trim_cr, int enc_mode, const uint8_t *lut256, int k, int complement_xor,
                                     int64_t n_bins, int hist_mode, int64_t *hist,
                                     int64_t *status, void *workspace, size_t workspace_bytes, void *stream);
+/*     Canonical minimizers: out[offsets[r] + j] = min over the window_size-k+1 k-mers i of window j of
+ *     min(h_i, hash of the reverse complement of k-mer i), with h_i and complement_xor as above.  A read and its reverse
+ *     complement give the same values (window j of one is window L - window_size - j of the other); window_size == k
+ *     gives the canonical k-mers.  The three entry points take the arguments of bnpk_rows_minimizers,
+ *     bnpk_rows_kmer_count and bnpk_chunk_kmer_count with complement_xor after window_size, and give their outputs.
+ *     Before any CUDA call: complement_xor outside 1..3 returns BNPK_E_BADARG, window_size < k or > 1024
+ *     BNPK_E_WINDOW, k outside 1..31 BNPK_E_K. */
+int bnpk_rows_minimizers_canonical(const uint8_t *base, size_t base_bytes, const int64_t *starts, const int32_t *lens,
+                                   size_t n_rows, int enc_mode, const uint8_t *lut256, int k, int window_size,
+                                   int complement_xor, const int64_t *offsets, int64_t *mins_out, int64_t *status,
+                                   void *stream);
+int bnpk_rows_minimizer_count_canonical(const uint8_t *base, size_t base_bytes, const int64_t *starts,
+                                        const int32_t *lens, size_t n_rows, int enc_mode, const uint8_t *lut256, int k,
+                                        int window_size, int complement_xor, int64_t n_bins, int hist_mode,
+                                        int64_t *hist, int64_t *status, void *stream);
+int bnpk_chunk_minimizer_count_canonical(const uint8_t *chunk, size_t n, size_t slice_begin, size_t slice_end,
+                                         int final_slice, int lines_per_entry, uint8_t header_char, int check_plus,
+                                         int trim_cr, int enc_mode, const uint8_t *lut256, int k, int window_size,
+                                         int complement_xor, int64_t n_bins, int hist_mode, int64_t *hist,
+                                         int64_t *status, void *workspace, size_t workspace_bytes, void *stream);
 
 /* K5  np.bincount(values % n_bins, minlength=n_bins) accumulated into hist
  *     (sequence/count_encoded.py:173-177; EncodedArray.__array_function__ encoded_array.py:459-460).
